@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — headline benchmark of the conversion path (contract in the task statement).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...] [--layout ...]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...] [--layout ...] [--dump-outputs DIR]
 
 A "step" = one ConversionPass::execute over the workload: BASELINE.json configs[1] — the SciFiHelmet stand-in
 (seeded displaced sphere, 70 074 triangles, 3 x 2048^2 RGBA8 maps; the Khronos asset is not available offline) at
@@ -237,6 +237,38 @@ def run_reference(args):
     print(json.dumps(line))
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_records(path: str, records: np.ndarray) -> None:
+    """--dump-outputs: the records of the last timed step (structured, _abi.record_dtype), one DIR/<field>.npy per record
+    field (one row per gaussian), and their count as DIR/total.npy.
+    The kernels append records in atomic arrival order, which differs from run to run, so rows are sorted by their
+    values (position first; the float bits mapped to integers that order like the floats, so -0.0 and NaN sort too).
+    PACKED56 stores opacity as logit(alpha), +inf for an opaque gaussian (as the reference's .ply writer does); it is
+    written as alpha.npy = sigmoid(opacity) in float64, finite and the form the parity tests compare it in.
+    Beyond DUMP_BYTES a fixed seeded sample of the sorted rows is kept."""
+    os.makedirs(path, exist_ok=True)
+    bits = records.view(np.int32).reshape(len(records), -1)
+    order = np.lexsort((bits ^ ((bits >> 31) & 0x7FFFFFFF)).T[::-1])
+    rows = records[order]
+    fields = {}
+    for name in rows.dtype.names:
+        if name == "opacity":
+            with np.errstate(over="ignore"):
+                fields["alpha"] = 1.0 / (1.0 + np.exp(-rows[name].astype(np.float64)))
+        else:
+            fields[name] = np.ascontiguousarray(rows[name])
+    row_bytes = sum(a.nbytes // max(1, len(a)) for a in fields.values())
+    keep = (DUMP_BYTES - 4096 * (len(fields) + 1)) // row_bytes
+    if len(rows) > keep:
+        pick = np.sort(np.random.default_rng(0).choice(len(rows), keep, replace=False))
+        fields = {k: v[pick] for k, v in fields.items()}
+    for name, a in fields.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
+    np.save(os.path.join(path, "total.npy"), np.array([len(records)], np.float64))
+
+
 def record_hashes(buf, n: int, stride: int, torch):
     """Order-independent fingerprint of n records: sorted per-record 64-bit hashes (device tensor)."""
     w = buf[: n * stride].view(torch.int32).view(n, stride // 4).to(torch.int64)
@@ -345,16 +377,26 @@ def run_ours(args):
             ms = float(t.item())
         return ms
 
+    def last_step(buf, n):
+        """rank 0, --dump-outputs: host copy of the records the last timed step wrote"""
+        if not args.dump_outputs or rank != 0:
+            return None
+        return buf[: n * stride].cpu().numpy().view(_abi.record_dtype(layout))
+
     clocks = ClockSampler(local) if rank == 0 else None
     gather_parity = None
     if world == 1:
         ms = run_timed(local_full)
         n_all = n_local = int(d_total.item())
+        dumped = last_step(out, n_all)
     else:
         ms_rep = run_timed(local_full)
         n_all = int(d_total.item())
+        dumped = last_step(out, n_all) if strategy == "replicate" else None
         ms_shard = run_timed(step_shard, pre=pg.barrier)
         torch.cuda.synchronize(dev)
+        if strategy == "shard":
+            dumped = last_step(pg.final, int(pg.total.item()))
         # untimed: the gathered buffer is the single-GPU multiset, on every rank
         n_g = int(pg.total.item())
         local_full()
@@ -467,6 +509,8 @@ def run_ours(args):
         dist.destroy_process_group()
     ds.free()
     ctx.close()
+    if dumped is not None:
+        dump_records(args.dump_outputs, dumped)
     if line is not None:
         print(json.dumps(line))
 
@@ -567,7 +611,13 @@ def main():
     ap.add_argument("--density", type=int, default=0, help="sampling density R (0 = the workload's BASELINE density)")
     ap.add_argument("--strategy", default="auto", choices=["auto", "shard", "replicate"],
                     help="N>1, device-resident leg: auto = shard.choose_strategy on live timings")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the records of the last timed step, sorted, as DIR/<field>.npy (PACKED56 opacity as alpha.npy) and their count as DIR/total.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's records (--impl ours)")
     args.warmup = max(3, args.warmup) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -1,5 +1,6 @@
 """CPU tests: pin the oracle against (a) golden vectors produced by the reference's own GLSL,
-(b) the live reference-shader build when present, (c) the analytic KATs of SURVEY.md 8c."""
+(b) what the reference build made of the inputs of the *live_reference* tests (tests/golden/ref_live_vectors.npz,
+tests/golden/make_golden_live.py), (c) the analytic KATs of SURVEY.md 8c."""
 from __future__ import annotations
 
 import os
@@ -12,11 +13,17 @@ from mesh2splat_b200 import _abi, synth
 from mesh2splat_b200._abi import LAYOUT_PACKED56, LAYOUT_REF96, Primitive, Scene
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_shader_vectors.npz")
+LIVE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_live_vectors.npz")
 
 
 @pytest.fixture(scope="module")
 def golden():
     return np.load(GOLDEN)
+
+
+@pytest.fixture(scope="module")
+def live():
+    return np.load(LIVE)
 
 
 def _same(a, b):  # bit-equal, NaN == NaN
@@ -57,17 +64,14 @@ def test_fragment_stage_matches_reference_fs_golden(golden):
     assert seen_discard
 
 
-@pytest.mark.skipif(oracle.ref_lib() is None, reason="oracle/_ref not built (no /root/reference on this box)")
-def test_triangle_stage_matches_live_reference_build():
-    rng = np.random.default_rng(7)
-    tris = synth.random_soup(500, seed=11, extent=3.0, tri_size=1.0)
-    mn = tris.reshape(-1, 3, 12)[:, :, :3].reshape(-1, 3).min(axis=0) - 0.1
-    mx = tris.reshape(-1, 3, 12)[:, :, :3].reshape(-1, 3).max(axis=0) + rng.random(3).astype(np.float32)
-    for t in tris:
-        glpos, scale, quat = oracle.ref_gs(t, mn, mx)
+def test_triangle_stage_matches_live_reference_build(live):
+    """500 triangles of a random soup (one bbox around all of them): converterGS.glsl's gl_Position.xy, Scale and
+    Quaternion as the reference build computed them, bit for bit."""
+    mn, mx = live["gs_bmin"], live["gs_bmax"]
+    for i, t in enumerate(live["gs_tris"]):
         s = oracle.triangle_setup(t, mn, mx, 256)
-        assert _same(np.array(s.ouv, np.float32) * np.float32(2) - np.float32(1), glpos[:, :2])
-        assert _same(np.array(s.scale, np.float32), scale) and _same(np.array(s.quat, np.float32), quat)
+        assert _same(np.array(s.ouv, np.float32) * np.float32(2) - np.float32(1), live["gs_glpos_xy"][i]), i
+        assert _same(np.array(s.scale, np.float32), live["gs_scale"][i]) and _same(np.array(s.quat, np.float32), live["gs_quat"][i]), i
 
 
 # ---- analytic KATs (SURVEY 8c) --------------------------------------------------------------------
@@ -217,74 +221,60 @@ def test_ply_bytes_match_reference_savePlyVector_golden(fmt):
     assert got == want
 
 
-def test_ply_bytes_match_live_reference_writer(tmp_path):
-    """Same check against the reference library itself when it is built here (fresh random records)."""
-    if oracle.ref_ply_lib() is None:
-        pytest.skip("oracle/_ref/libm2s_refply.so not built (no /root/reference on this machine)")
-    rng = np.random.default_rng(77)
-    rec = rng.random((500, 24)).astype(np.float32)
-    rec[:, 8:11] *= np.float32(0.01); rec[:50, 7] = 1.0
-    mult = float(np.float32(0.65) / np.float32(300))
+def test_ply_bytes_match_live_reference_writer(live):
+    """Same check on other records (uniform random, small scales, some alpha 1) and another multiplier: the files the
+    reference's savePlyVector wrote for them, byte for byte."""
+    rec = live["ply_records"]
+    mult = float(live["ply_scale_multiplier"])
     for fmt in (0, 1, 2):
-        path = tmp_path / f"live{fmt}.ply"
-        assert oracle.ref_save_ply(str(path), rec, fmt, mult)
-        assert path.read_bytes() == oracle.ply_bytes(rec.view(_abi.record_dtype(LAYOUT_REF96)).reshape(-1), fmt, mult)
+        assert live[f"ply_format_{fmt}"].tobytes() == oracle.ply_bytes(rec.view(_abi.record_dtype(LAYOUT_REF96)).reshape(-1), fmt, mult)
 
 
-def test_loader_matches_live_reference_parser(tmp_path):
-    """Fresh random node transforms / attribute combinations through the reference's own parser (when it is built
-    here) and through m2s_glb_load: bit-identical triangle data."""
-    if oracle.ref_loader_lib() is None:
-        pytest.skip("oracle/_ref/libm2s_refloader.so not built (no /root/reference on this machine)")
-    import sys
-    sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+def test_loader_matches_live_reference_parser(tmp_path, live):
+    """Random node transforms / attribute combinations (util.loader_transform_cases) through m2s_glb_load: the
+    triangle data the reference's own parser produced for the same files, bit for bit."""
     from test_abi_host import _make_glb
+    from util import loader_transform_cases
     from mesh2splat_b200.gltf import load_glb
-    rng = np.random.default_rng(99)
-    for k in range(24):
-        if k % 2 == 0:
-            M = np.eye(4, dtype=np.float32); M[:3, :3] = rng.normal(size=(3, 3)); M[:3, 3] = rng.normal(size=3) * 5
-            kw = dict(matrix=M)
-        else:
-            q = rng.normal(size=4); q /= np.linalg.norm(q)
-            kw = dict(trs=([float(v) for v in rng.normal(size=3)], [float(v) for v in q], [float(v) for v in rng.random(3) * 2 + 0.2]))
-        kw.update(with_normals=bool(k % 3), with_tangents=bool(k % 5), indexed=bool(k % 4))
+    cases = loader_transform_cases()
+    counts = live["loader_face_counts"]
+    assert len(counts) == len(cases)
+    wants = np.split(live["loader_faces"], np.cumsum(counts)[:-1])
+    for k, kw in enumerate(cases):
         p = tmp_path / f"c{k}.glb"
         _make_glb(str(p), **kw)
-        ok, meshes = oracle.ref_load_glb(str(p))
         s = load_glb(str(p))
-        want = np.vstack([m["faces"] for m in meshes])
-        assert ok and np.array_equal(want.view(np.uint32), s.triangles.view(np.uint32)), k
+        assert wants[k].shape == s.triangles.shape and np.array_equal(wants[k].view(np.uint32), s.triangles.view(np.uint32)), k
 
 
-def test_loader_matches_live_reference_parser_on_random_scene_graphs(tmp_path):
+def test_loader_matches_live_reference_parser_on_random_scene_graphs(tmp_path, live):
     """Differential test on 120 random multi-mesh .glb files (util.make_complex_glb): nested matrix / TRS nodes,
-    instanced meshes, shared images, every index type, skipped primitives, two scenes — m2s_glb_load vs the
-    reference's own parser: identical triangles (bitwise), names, base colours, texture slots and texels."""
-    if oracle.ref_loader_lib() is None:
-        pytest.skip("oracle/_ref/libm2s_refloader.so not built (no /root/reference on this machine)")
-    import sys
-    sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
-    from util import make_complex_glb
+    instanced meshes, shared images, every index type, skipped primitives, two scenes — m2s_glb_load vs what the
+    reference's own parser made of them: identical triangles (bitwise), names, base colours, texture slots and texels
+    (triangles and texels through their recorded SHA-256 digests)."""
+    from util import array_digest, make_complex_glb
     from mesh2splat_b200.gltf import load_glb
+    seeds = [int(x) for x in live["graph_seeds"]]
+    first = np.concatenate([[0], np.cumsum(live["graph_mesh_counts"])])
     compared = 0
     for seed in range(5000, 5120):
         p = tmp_path / "g.glb"
         make_complex_glb(str(p), seed)
-        ok, meshes = oracle.ref_load_glb(str(p))
-        if not ok or not meshes:
+        if seed not in seeds:   # the reference rejects the file or finds no mesh in it
             continue
+        j = seeds.index(seed)
+        m0, m1 = int(first[j]), int(first[j + 1])
         s = load_glb(str(p))
-        want = np.vstack([m["faces"] for m in meshes])
-        assert want.shape == s.triangles.shape and np.array_equal(want.view(np.uint32), s.triangles.view(np.uint32)), seed
-        assert [m["name"] for m in meshes] == [q.name for q in s.primitives], seed
-        for m, q in zip(meshes, s.primitives):
-            assert np.array_equal(m["base_color"], np.asarray(q.base_color_factor, np.float32)), seed
+        assert array_digest([s.triangles]) == live["graph_faces_sha256"][j], seed
+        assert [str(x) for x in live["graph_mesh_names"][m0:m1]] == [q.name for q in s.primitives], seed
+        texels = []
+        for q, bc, present in zip(s.primitives, live["graph_base_color"][m0:m1], live["graph_tex_present"][m0:m1]):
+            assert np.array_equal(bc, np.asarray(q.base_color_factor, np.float32)), seed
             for which, idx in ((0, q.albedo_texture), (1, q.normal_texture), (2, q.metallic_roughness_texture)):
-                t = m["textures"].get(which)
-                assert (t is None) == (idx < 0), (seed, q.name, which)
-                if t is not None:
-                    assert np.array_equal(t, s.textures[idx]), (seed, q.name, which)
+                assert bool(present[which]) == (idx >= 0), (seed, q.name, which)
+                if idx >= 0:
+                    texels.append(s.textures[idx])
+        assert array_digest(texels) == live["graph_texels_sha256"][j], seed
         compared += 1
     assert compared >= 100
 
@@ -313,18 +303,17 @@ def test_prepass_oracle_matches_reference_shader_golden_vectors():
     assert n == 5
 
 
-def test_prepass_live_reference_build_when_available():
-    """Where oracle/_ref/libm2s_refprepass.so exists (the build container), run the reference shader live on fresh seeds."""
-    if oracle.ref_prepass_lib() is None:
-        pytest.skip("oracle/_ref/libm2s_refprepass.so not built (no /root/reference on this box)")
+def test_prepass_live_reference_build_when_available(live):
+    """The golden cameras and formats on other gaussians (64 of each case, moved by up to 0.15): the reference shader's
+    outputs for them, recorded by tests/golden/make_golden_live.py."""
     from util import assert_prepass_match
-    rng = np.random.default_rng(77)
-    for c in _prepass_golden():
-        g = c["gaussians"].copy()
-        g[:, 0:3] += (rng.random((len(g), 3)).astype(np.float32) - 0.5) * 0.3
-        args = (g, c["view"], c["proj"], c["model"], c["resolution"], c["near_far"], c["std_dev"], c["render_mode"], c["fmt"], 0)
-        a, b = oracle.prepass(*args), oracle.ref_prepass(*args)
-        assert_prepass_match(a[0], a[1], b[0], b[1], c["resolution"], ordered=True)
+    n = 0
+    for i, c in enumerate(_prepass_golden()):
+        g = live[f"prepass_g{i}"]
+        a = oracle.prepass(g, c["view"], c["proj"], c["model"], c["resolution"], c["near_far"], c["std_dev"], c["render_mode"], c["fmt"], 0)
+        assert_prepass_match(a[0], a[1], live[f"prepass_quads{i}"], live[f"prepass_depths{i}"], c["resolution"], ordered=True)
+        n += len(a[0])
+    assert n > 0
 
 
 def test_packed56_decodes_to_the_gaussian_vertex_it_was_encoded_from():

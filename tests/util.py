@@ -328,6 +328,35 @@ def make_complex_glb(path: str, seed: int) -> None:
         f.write(struct.pack("<I4s", len(binblob), b"BIN\x00")); f.write(binblob)
 
 
+def loader_transform_cases(n: int = 24, seed: int = 99) -> list:
+    """Keyword arguments of test_abi_host._make_glb for n quads under random node transforms (even k: a `matrix` node,
+    odd k: TRS) and varying attribute sets.  Shared by the loader test and tests/golden/make_golden_live.py."""
+    rng = np.random.default_rng(seed)
+    cases = []
+    for k in range(n):
+        if k % 2 == 0:
+            M = np.eye(4, dtype=np.float32); M[:3, :3] = rng.normal(size=(3, 3)); M[:3, 3] = rng.normal(size=3) * 5
+            kw = dict(matrix=M)
+        else:
+            q = rng.normal(size=4); q /= np.linalg.norm(q)
+            kw = dict(trs=([float(v) for v in rng.normal(size=3)], [float(v) for v in q], [float(v) for v in rng.random(3) * 2 + 0.2]))
+        kw.update(with_normals=bool(k % 3), with_tangents=bool(k % 5), indexed=bool(k % 4))
+        cases.append(kw)
+    return cases
+
+
+def array_digest(arrays) -> str:
+    """SHA-256 over the shapes, dtypes and bytes of a sequence of arrays: equal digests <=> equal arrays (for golden
+    data too large to store whole)."""
+    import hashlib
+    h = hashlib.sha256()
+    for a in arrays:
+        a = np.ascontiguousarray(a)
+        h.update(f"{a.dtype.str}{a.shape};".encode())
+        h.update(a.tobytes())
+    return h.hexdigest()
+
+
 # ---- viewer prepass (SURVEY 8 f-4) --------------------------------------------------------------------------------
 def assert_prepass_match(got_quads, got_depths, want_quads, want_depths, resolution, ordered: bool):
     """QuadNdcTransformation arrays [n, 24] + view depths.  ordered = False: the GPU appends in atomic arrival order, both
