@@ -18,6 +18,14 @@
  *      src/parsers/parsers.cpp:232-316,339-428,431-514,631-651)
  *   SceneManager::loadModel -> execute -> exportPly             m2s_convert_file
  *     (src/utils/SceneManager.hpp:18-20)
+ *   RadixSortPass::execute + radixSortPrepass.glsl              m2s_sort_quads, m2s_sort_quads_enqueue
+ *     + radixSortGather.glsl + glu::RadixSort
+ *     (src/renderer/renderPasses/RadixSortPass.cpp:8-90,
+ *      thirdParty/RadixSort.hpp:1393-1530)
+ *   GaussianSplattingPass::execute + gaussianSplatting{VS,PS}   m2s_splat, m2s_splat_enqueue
+ *     .glsl into the G-buffer
+ *     (src/renderer/renderPasses/GaussianSplattingPass.cpp:37-97,
+ *      src/renderer/renderer.cpp:329-379)
  *
  * Plain pointers and sizes only; no C++/torch types.  All functions return an
  * m2s_status; m2s_last_error() gives the thread-local message of the last
@@ -148,8 +156,9 @@ void m2s_params_default(m2s_params* p);
 m2s_status m2s_ctx_create(int device, m2s_ctx** out);
 void m2s_ctx_destroy(m2s_ctx* ctx);
 int m2s_ctx_device(const m2s_ctx* ctx);
-/* Conditions raised on the device that an enqueue-only call cannot return (a fused-gather wait that timed out after
- * 2 s because a peer never published): M2S_OK or M2S_E_CUDA; clears the condition.  Call after synchronising. */
+/* Conditions raised on the device that an enqueue-only call cannot return: a fused-gather wait that timed out after
+ * 2 s because a peer never published (M2S_E_CUDA), or an m2s_splat_enqueue whose quads touched more (tile, quad) pairs
+ * than its max_pairs (M2S_E_CAPACITY).  M2S_OK if neither; clears the condition.  Call after synchronising. */
 m2s_status m2s_ctx_status(m2s_ctx* ctx);
 int m2s_ctx_sm_count(const m2s_ctx* ctx);
 
@@ -275,7 +284,8 @@ typedef struct m2s_prepass_params {
     float resolution[2];       /* renderContext.rendererResolution */
     float near_far[2];
     float std_dev;             /* gaussianStd / resolutionTarget (GaussiansPrepass.cpp:18) */
-    uint32_t render_mode;      /* 0 (or 6) colour, 1 depth, 2 normal */
+    uint32_t render_mode;      /* 0 (or 6) colour, 1 depth, 2 normal; 4, 5: colour and opacity 0 (the shader's if-chain
+                                  sets none), for the splatting pass's overdraw and metallic-roughness modes */
     uint32_t layout;           /* M2S_LAYOUT_REF96 or M2S_LAYOUT_PACKED56 */
     uint32_t reserved;
 } m2s_prepass_params;
@@ -289,6 +299,58 @@ m2s_status m2s_prepass_enqueue(m2s_ctx* ctx, const void* d_records, uint64_t cou
 /* Synchronous variant on the context stream; *valid receives the counter. */
 m2s_status m2s_prepass(m2s_ctx* ctx, const void* d_records, uint64_t count, const m2s_prepass_params* params,
                        void* d_quads, float* d_depths, uint32_t* valid);
+
+/* ---- the passes after the prepass: depth sort (SURVEY 8 f-5) and splatting into the G-buffer (f-6) ----------------
+ * RadixSortPass::execute (src/renderer/renderPasses/RadixSortPass.cpp:8-90, radixSortPrepass.glsl, radixSortGather.glsl,
+ * thirdParty/RadixSort.hpp:1393-1530): key = floatBitsToUint(view depth) with no sign fix-up, value = prepass index;
+ * the stable ascending order of the 32-bit keys over the prepass arrival order (survivors have negative view z: nearest
+ * first); the gather moves each 96-byte quad to its sorted place.  d_count (optional): the prepass's d_valid, a device
+ * count that overrides `count` downwards, so convert -> prepass -> sort -> splat needs no host round trip.  d_order
+ * (optional) receives the prepass index of every sorted quad.  Scratch comes from the context's stream-ordered pool. */
+m2s_status m2s_sort_quads_enqueue(m2s_ctx* ctx, const void* d_quads, const float* d_depths, uint64_t count,
+                                  const uint32_t* d_count, void* d_sorted_quads, uint32_t* d_order, void* stream);
+/* Synchronous variant on the context stream; device_ms (optional) receives the device time. */
+m2s_status m2s_sort_quads(m2s_ctx* ctx, const void* d_quads, const float* d_depths, uint64_t count, void* d_sorted_quads,
+                          uint32_t* d_order, float* device_ms);
+
+/* GaussianSplattingPass::execute (GaussianSplattingPass.cpp:37-97) + gaussianSplattingVS.glsl + gaussianSplattingPS.glsl
+ * into the 5-target G-buffer of Renderer::createGBuffer (renderer.cpp:329-379): every sorted quad is two triangles over
+ * the corners (-1,-1), (-1,1), (1,1), (1,-1), rasterised into a width x height viewport with no depth test and no culling;
+ * per fragment g = exp(-0.5 a dx^2 - 0.5 c dy^2 - b dx dy) and
+ *   position = (wsPos, 1) g               RGBA16F
+ *   normal   = (normal, opacity) g        RGBA16F
+ *   albedo   = (rgb a, a) g               RGBA8    (render mode 4, overdraw: (.01, .005, 0, .01))
+ *   depth    = (d, d, d, a g), d = z g    RGBA16F
+ *   metallic_roughness = (m, r, 0, 1) g   RGBA8
+ * blended front to back with ONE_MINUS_DST_ALPHA, ONE per target (mode 4: ONE, ONE) and converted to the storage format
+ * after every fragment; the targets start cleared to 0.  Choices GL leaves to the implementation are listed in DESIGN.md
+ * section 2.  Not reproduced: mode 3 (debug colours of the prepass) and the lighting of mode 6 (which writes the same
+ * G-buffer as mode 0). */
+typedef struct m2s_splat_params {
+    uint32_t width, height;   /* renderContext.rendererResolution: 1..4096 each */
+    uint32_t render_mode;     /* 0, 1, 2, 4, 5 or 6 */
+    uint32_t reserved;
+} m2s_splat_params;
+/* Device images, row-major, row 0 = the bottom row (GL's window origin, as glReadPixels returns it).  position, normal and
+ * depth hold half4 per pixel, albedo and metallic_roughness uchar4; every pointer 16-byte aligned. */
+typedef struct m2s_gbuffer {
+    void* position;
+    void* normal;
+    void* albedo;
+    void* depth;
+    void* metallic_roughness;
+} m2s_gbuffer;
+/* Non-lit composite of the deferred pass (gaussianSplattingDeferredPS.glsl:120-131) is a read of one target: mode 5 shows
+ * (metallic_roughness.rg, 0, 1), every other mode but 6 (albedo.rgb, 1). */
+/* Enqueue-only: d_sorted_quads holds `count` x 96 B (d_count as for the sort).  max_pairs: capacity of the (tile, quad) pair
+ * scratch, 16 x 16 pixel tiles; the radix sort of the pairs runs over all max_pairs entries.  If the quads touch more
+ * pairs, the G-buffer is left cleared and m2s_ctx_status reports M2S_E_CAPACITY. */
+m2s_status m2s_splat_enqueue(m2s_ctx* ctx, const void* d_sorted_quads, uint64_t count, const uint32_t* d_count,
+                             const m2s_splat_params* params, const m2s_gbuffer* gbuffer, uint64_t max_pairs, void* stream);
+/* Synchronous variant on the context stream: counts the pairs, reads the count back and sizes the scratch exactly.
+ * pairs and device_ms (both optional) receive the pair count and the device time of the pass. */
+m2s_status m2s_splat(m2s_ctx* ctx, const void* d_sorted_quads, uint64_t count, const uint32_t* d_count,
+                     const m2s_splat_params* params, const m2s_gbuffer* gbuffer, uint64_t* pairs, float* device_ms);
 
 #ifdef __cplusplus
 }

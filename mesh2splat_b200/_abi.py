@@ -63,6 +63,22 @@ class m2s_prepass_params(C.Structure):
 
 
 QUAD_BYTES = 96
+MAX_SPLAT_SIZE = 4096
+
+
+class m2s_splat_params(C.Structure):
+    """include/m2s.h: viewport and render mode of GaussianSplattingPass::execute."""
+    _fields_ = [("width", C.c_uint32), ("height", C.c_uint32), ("render_mode", C.c_uint32), ("reserved", C.c_uint32)]
+
+
+class m2s_gbuffer(C.Structure):
+    """include/m2s.h: the five G-buffer images (device pointers, row-major, row 0 = bottom row)."""
+    _fields_ = [("position", C.c_void_p), ("normal", C.c_void_p), ("albedo", C.c_void_p), ("depth", C.c_void_p),
+                ("metallic_roughness", C.c_void_p)]
+
+
+# G-buffer targets: (name, storage) as Renderer::createGBuffer (renderer.cpp:329-379) allocates them
+GBUFFER_TARGETS = (("position", "f16"), ("normal", "f16"), ("albedo", "u8"), ("depth", "f16"), ("metallic_roughness", "u8"))
 
 
 def make_prepass_params(world_to_view, view_to_clip, model_to_world, resolution, near_far, std_dev: float, render_mode: int, layout: int):

@@ -20,6 +20,7 @@ SYMBOLS = [
     "m2s_ply_header", "m2s_ply_encode", "m2s_ply_write", "m2s_convert_file",
     "m2s_glb_load", "m2s_hscene_view", "m2s_hscene_primitive_name", "m2s_hscene_free",
     "m2s_prepass", "m2s_prepass_enqueue",
+    "m2s_sort_quads", "m2s_sort_quads_enqueue", "m2s_splat", "m2s_splat_enqueue",
 ]
 
 
@@ -106,6 +107,14 @@ def lib() -> C.CDLL:
     L.m2s_prepass_enqueue.argtypes = [vp, vp, u64, vp, C.POINTER(_abi.m2s_prepass_params), vp, vp, vp, vp]
     L.m2s_prepass.restype = i32
     L.m2s_prepass.argtypes = [vp, vp, u64, C.POINTER(_abi.m2s_prepass_params), vp, vp, C.POINTER(u32)]
+    L.m2s_sort_quads_enqueue.restype = i32
+    L.m2s_sort_quads_enqueue.argtypes = [vp, vp, vp, u64, vp, vp, vp, vp]
+    L.m2s_sort_quads.restype = i32
+    L.m2s_sort_quads.argtypes = [vp, vp, vp, u64, vp, vp, C.POINTER(f32)]
+    L.m2s_splat_enqueue.restype = i32
+    L.m2s_splat_enqueue.argtypes = [vp, vp, u64, vp, C.POINTER(_abi.m2s_splat_params), C.POINTER(_abi.m2s_gbuffer), u64, vp]
+    L.m2s_splat.restype = i32
+    L.m2s_splat.argtypes = [vp, vp, u64, vp, C.POINTER(_abi.m2s_splat_params), C.POINTER(_abi.m2s_gbuffer), C.POINTER(u64), C.POINTER(f32)]
     _lib = L
     return L
 

@@ -80,6 +80,49 @@ class ConvertOutput:
         return None if self.keys is None else self.keys[: self.written].cpu().numpy().view(np.uint64)
 
 
+@dataclass
+class GBuffer:
+    """The five targets of GaussianSplattingPass (renderer.cpp:329-379) as torch device tensors of shape (height, width, 4),
+    row 0 = the bottom row (GL's window origin): position, normal, depth float16; albedo, metallic_roughness uint8."""
+    position: object
+    normal: object
+    albedo: object
+    depth: object
+    metallic_roughness: object
+    render_mode: int
+    pairs: int = 0              # (tile, quad) pairs the splat walked
+    device_ms: float = 0.0      # device time of the splatting pass
+    survivors: int = 0          # quads splatted (Context.render: the prepass's count)
+
+    @staticmethod
+    def empty(width: int, height: int, render_mode: int, device) -> "GBuffer":
+        torch = _torch()
+        mk = {"f16": lambda: torch.empty((height, width, 4), dtype=torch.float16, device=device),
+              "u8": lambda: torch.empty((height, width, 4), dtype=torch.uint8, device=device)}
+        return GBuffer(*[mk[kind]() for _, kind in _abi.GBUFFER_TARGETS], render_mode=render_mode)
+
+    def c_struct(self) -> _abi.m2s_gbuffer:
+        return _abi.m2s_gbuffer(*[getattr(self, name).data_ptr() for name, _ in _abi.GBUFFER_TARGETS])
+
+    def numpy(self) -> dict:
+        """{target name: numpy array (height, width, 4)}: float16 or uint8."""
+        return {name: getattr(self, name).cpu().numpy() for name, _ in _abi.GBUFFER_TARGETS}
+
+    def image(self, mode: int | None = None) -> np.ndarray:
+        """The non-lit composite of the deferred pass (gaussianSplattingDeferredPS.glsl:120-131), float32 (height, width, 4):
+        mode 5 shows (metallic_roughness.rg, 0, 1), every other mode (albedo.rgb, 1).  Mode 6 (lighting) is not provided."""
+        mode = self.render_mode if mode is None else mode
+        if mode == 6:
+            raise ValueError("render mode 6 needs the lighting of the deferred pass, which is not provided")
+        src = (self.metallic_roughness if mode == 5 else self.albedo).cpu().numpy().astype(np.float32) / np.float32(255.0)
+        out = np.zeros(src.shape, np.float32)
+        out[..., 3] = 1.0
+        out[..., 0:2] = src[..., 0:2]
+        if mode != 5:
+            out[..., 2] = src[..., 2]
+        return out
+
+
 class Context:
     """One per GPU (m2s_ctx)."""
 
@@ -173,6 +216,77 @@ class Context:
         check(lib().m2s_prepass(self.handle, records.data_ptr(), count, C.byref(p), quads.data_ptr(), depths.data_ptr(), C.byref(valid)))
         m = int(valid.value)
         return quads[: m * _abi.QUAD_BYTES].cpu().numpy().view(np.float32).reshape(m, 24).copy(), depths[:m].cpu().numpy().copy()
+
+    def sort_quads(self, quads, depths, count: int, d_count=None, order: bool = True):
+        """RadixSortPass on device-resident prepass output (torch tensors: quads uint8/float32 of count x 96 B, depths float32):
+        the stable ascending order of floatBitsToUint(depth).  d_count: optional int32 device tensor (the prepass's counter)
+        that overrides `count` downwards.  Returns (sorted quads as a float32 tensor [count, 24], prepass index of each
+        sorted quad as an int32 tensor [count] or None); with d_count only the first *d_count rows are defined."""
+        torch = _torch()
+        dev = quads.device
+        torch.cuda.current_stream(dev).synchronize()   # inputs made on torch's stream; the sort runs on the context stream
+        sorted_q = torch.empty((max(1, count), 24), dtype=torch.float32, device=dev)
+        idx = torch.empty(max(1, count), dtype=torch.int32, device=dev) if order else None
+        check(lib().m2s_sort_quads_enqueue(self.handle, quads.data_ptr(), depths.data_ptr(), count,
+                                           d_count.data_ptr() if d_count is not None else None, sorted_q.data_ptr(),
+                                           idx.data_ptr() if idx is not None else None, None))
+        self.synchronize()
+        return sorted_q[:count], (idx[:count] if idx is not None else None)
+
+    def splat(self, sorted_quads, count: int, width: int, height: int, render_mode: int = 0, d_count=None,
+              max_pairs: int | None = None) -> GBuffer:
+        """GaussianSplattingPass into a fresh G-buffer.  max_pairs None: m2s_splat (counts the pairs and sizes the scratch
+        exactly; reports pairs and device time); else m2s_splat_enqueue with that pair capacity, then a synchronise and
+        m2s_ctx_status (raises M2SError with M2S_E_CAPACITY if the quads touch more pairs: the G-buffer is then cleared)."""
+        torch = _torch()
+        dev = sorted_quads.device
+        torch.cuda.current_stream(dev).synchronize()
+        gb = GBuffer.empty(width, height, render_mode, dev)
+        gb.survivors = count
+        p = _abi.m2s_splat_params(width, height, render_mode, 0)
+        g = gb.c_struct()
+        dc = d_count.data_ptr() if d_count is not None else None
+        if max_pairs is None:
+            pairs, ms = C.c_uint64(0), C.c_float(0)
+            check(lib().m2s_splat(self.handle, sorted_quads.data_ptr(), count, dc, C.byref(p), C.byref(g), C.byref(pairs), C.byref(ms)))
+            gb.pairs, gb.device_ms = int(pairs.value), float(ms.value)
+        else:
+            check(lib().m2s_splat_enqueue(self.handle, sorted_quads.data_ptr(), count, dc, C.byref(p), C.byref(g), max_pairs, None))
+            self.synchronize()
+            check(lib().m2s_ctx_status(self.handle))
+        return gb
+
+    def render(self, records, count: int, layout: int, world_to_view, view_to_clip, model_to_world, width: int, height: int,
+               std_dev: float, render_mode: int = 0, near_far=(0.01, 100.0)) -> GBuffer:
+        """prepass -> sort -> splat on the context stream (GaussiansPrepass, RadixSortPass, GaussianSplattingPass): the
+        records (e.g. ConvertOutput.data) seen by the camera at width x height.  The prepass's counter feeds the sort and
+        the splat on the device; the only host round trip is the splat's pair count."""
+        torch = _torch()
+        dev = records.device
+        torch.cuda.current_stream(dev).synchronize()
+        n = max(1, count)
+        quads = torch.empty(n * _abi.QUAD_BYTES, dtype=torch.uint8, device=dev)
+        depths = torch.empty(n, dtype=torch.float32, device=dev)
+        valid = torch.empty(1, dtype=torch.int32, device=dev)
+        sorted_q = torch.empty(n * _abi.QUAD_BYTES, dtype=torch.uint8, device=dev)
+        p = _abi.make_prepass_params(world_to_view, view_to_clip, model_to_world, (width, height), near_far, std_dev, render_mode,
+                                     layout)
+        L = lib()
+        check(L.m2s_prepass_enqueue(self.handle, records.data_ptr(), count, None, C.byref(p), quads.data_ptr(), depths.data_ptr(),
+                                    valid.data_ptr(), None))
+        check(L.m2s_sort_quads_enqueue(self.handle, quads.data_ptr(), depths.data_ptr(), count, valid.data_ptr(),
+                                       sorted_q.data_ptr(), None, None))
+        gb = GBuffer.empty(width, height, render_mode, dev)
+        sp = _abi.m2s_splat_params(width, height, render_mode, 0)
+        g = gb.c_struct()
+        pairs, ms = C.c_uint64(0), C.c_float(0)
+        check(L.m2s_splat(self.handle, sorted_q.data_ptr(), count, valid.data_ptr(), C.byref(sp), C.byref(g), C.byref(pairs), C.byref(ms)))
+        gb.pairs, gb.device_ms, gb.survivors = int(pairs.value), float(ms.value), int(valid.item())
+        return gb
+
+    def synchronize(self) -> None:
+        """Waits for the context stream (through a device-wide synchronise: the stream is not exposed)."""
+        _torch().cuda.synchronize(self.device)
 
     def convert_timed(self, dscene: DeviceScene, params: _abi.m2s_params, out, capacity: int):
         """One conversion with an event between the two kernels (they do not overlap): (raster_ms, fragment_ms)."""
@@ -304,5 +418,5 @@ class ConversionPass:
         rc.lastResult = out
 
 
-__all__ = ["Context", "DeviceScene", "ConvertOutput", "RenderContext", "SceneManager", "ConversionPass",
+__all__ = ["Context", "DeviceScene", "ConvertOutput", "GBuffer", "RenderContext", "SceneManager", "ConversionPass",
            "ply_header", "ply_write", "M2SError"]

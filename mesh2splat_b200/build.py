@@ -14,8 +14,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libm2s.so")
-SOURCES = ["m2s_kernels.cu", "m2s_prepass.cu", "m2s_api.cu", "m2s_host.cpp", "m2s_glb.cpp"]
-HEADERS = ["m2s_device.cuh", "m2s_prepass.cuh", os.path.join("..", "..", "include", "m2s.h")]
+SOURCES = ["m2s_kernels.cu", "m2s_prepass.cu", "m2s_render.cu", "m2s_api.cu", "m2s_host.cpp", "m2s_glb.cpp"]
+HEADERS = ["m2s_device.cuh", "m2s_prepass.cuh", "m2s_render.cuh", "m2s_span.cuh", os.path.join("..", "..", "include", "m2s.h")]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 
 

@@ -13,6 +13,7 @@
 #include "../../include/m2s.h"
 #include "m2s_device.cuh"
 #include "m2s_prepass.cuh"
+#include "m2s_render.cuh"
 
 namespace m2s {
 int convert_warps_per_cta(int layout);
@@ -66,6 +67,7 @@ struct m2s_ctx {
     uint32_t* h_status = nullptr;            // pinned + mapped: raised by device-side waits that timed out (fused gather)
     uint32_t* d_status = nullptr;            // its device view
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev_mid = nullptr;
+    cudaEvent_t ev_r[4] = {};                // timing of the synchronous sort / splat (created on first use)
     // convert_host pipeline: a second stream for the downloads, per-chunk counts and events
     static constexpr int kMaxChunks = 8;
     cudaStream_t stream2 = nullptr;
@@ -251,6 +253,7 @@ M2S_EXPORT void m2s_ctx_destroy(m2s_ctx* c) {
     for (auto& v : c->vr) { if (v.d_minmax) cudaFree(v.d_minmax); if (v.h_minmax) cudaFreeHost(v.h_minmax); if (v.ev) cudaEventDestroy(v.ev); }
     for (int i = 0; i < m2s_ctx::kMaxChunks; ++i) if (c->ev_chunk[i]) cudaEventDestroy(c->ev_chunk[i]);
     cudaEventDestroy(c->ev0); cudaEventDestroy(c->ev1); if (c->ev_mid) cudaEventDestroy(c->ev_mid);
+    for (cudaEvent_t e : c->ev_r) if (e) cudaEventDestroy(e);
     if (c->stream2) cudaStreamDestroy(c->stream2);
     if (c->stream3) cudaStreamDestroy(c->stream3);
     if (c->stream4) cudaStreamDestroy(c->stream4);
@@ -268,6 +271,10 @@ M2S_EXPORT m2s_status m2s_ctx_status(m2s_ctx* c) {
     if (!c) { set_error("m2s_ctx_status: ctx is NULL"); return M2S_E_INVALID; }
     const uint32_t v = __atomic_exchange_n(c->h_status, 0u, __ATOMIC_ACQ_REL);
     if (v == 0) return M2S_OK;
+    if (v == kStatusSplatCapacity) {
+        set_error("m2s_splat_enqueue: the quads touch more (tile, quad) pairs than max_pairs; the G-buffer was left cleared");
+        return M2S_E_CAPACITY;
+    }
     c->dirty = true;
     set_error(std::string("fused gather: a peer rank did not publish its ") + ((v & 1u) ? "count" : "completion flag") +
               " within 2 s (did every rank call m2s_convert_gather_enqueue the same number of times?)");
@@ -1082,7 +1089,7 @@ M2S_EXPORT m2s_status m2s_prepass_enqueue(m2s_ctx* ctx, const void* d_records, u
                                           const m2s_prepass_params* p, void* d_quads, float* d_depths, uint32_t* d_valid, void* stream_) {
     if (!ctx || !p || !d_valid || (count && (!d_records || !d_quads || !d_depths))) { set_error("m2s_prepass: NULL argument"); return M2S_E_INVALID; }
     if (p->layout != M2S_LAYOUT_REF96 && p->layout != M2S_LAYOUT_PACKED56) { set_error("m2s_prepass: layouts REF96 and PACKED56 only"); return M2S_E_INVALID; }
-    if (p->render_mode == 3 || (p->render_mode > 2 && p->render_mode != 6)) { set_error("m2s_prepass: render modes 0 (6), 1 and 2 only"); return M2S_E_INVALID; }
+    if (p->render_mode == 3 || p->render_mode > 6) { set_error("m2s_prepass: render modes 0-2 and 4-6 only"); return M2S_E_INVALID; }
     if (count >= (1ull << 32)) { set_error("m2s_prepass: too many gaussians (< 2^32 supported)"); return M2S_E_INVALID; }
     if ((reinterpret_cast<uintptr_t>(d_quads) & 15u) || (reinterpret_cast<uintptr_t>(d_records) & 15u)) {
         set_error("m2s_prepass: the record and quad buffers must be 16-byte aligned"); return M2S_E_INVALID;
@@ -1127,5 +1134,171 @@ M2S_EXPORT m2s_status m2s_prepass(m2s_ctx* ctx, const void* d_records, uint64_t 
     CUDA_TRY(cudaMemcpyAsync(&v, ctx->d_prepass_valid, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     if (valid) *valid = v;
+    return M2S_OK;
+}
+
+// ---- depth sort (SURVEY 8 f-5) and splatting pass (f-6): RadixSortPass + GaussianSplattingPass ----------------------
+static inline bool misaligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) != 0; }
+
+static m2s_status timing_events(m2s_ctx* ctx) {
+    for (cudaEvent_t& e : ctx->ev_r)
+        if (!e) CUDA_TRY(cudaEventCreate(&e));
+    return M2S_OK;
+}
+
+M2S_EXPORT m2s_status m2s_sort_quads_enqueue(m2s_ctx* ctx, const void* d_quads, const float* d_depths, uint64_t count,
+                                             const uint32_t* d_count, void* d_sorted_quads, uint32_t* d_order, void* stream_) {
+    if (!ctx || (count && (!d_quads || !d_depths || !d_sorted_quads))) { set_error("m2s_sort_quads: NULL argument"); return M2S_E_INVALID; }
+    if (count >= (1ull << 32)) { set_error("m2s_sort_quads: too many quads (< 2^32 supported)"); return M2S_E_INVALID; }
+    if (misaligned16(d_quads) || misaligned16(d_sorted_quads) || misaligned16(d_depths) || misaligned16(d_order)) {
+        set_error("m2s_sort_quads: every buffer must be 16-byte aligned"); return M2S_E_INVALID;
+    }
+    if (count == 0) return M2S_OK;
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    cudaStream_t stream = stream_ ? (cudaStream_t)stream_ : ctx->stream;
+    SortArgs a;
+    std::memset(&a, 0, sizeof(a));
+    a.quads = (const float4*)d_quads; a.depths = d_depths; a.count = count; a.d_count = d_count;
+    a.sorted = (float4*)d_sorted_quads; a.order = d_order;
+    a.temp_bytes = sort_temp_bytes(count);
+    const size_t n4 = ((size_t)count * 4 + 255) & ~(size_t)255;   // 256-byte aligned sub-buffers
+    unsigned char* scratch = nullptr;
+    CUDA_TRY(cudaMallocAsync((void**)&scratch, 4 * n4 + a.temp_bytes, stream));   // the context's stream-ordered pool
+    a.keys[0] = (uint32_t*)scratch; a.keys[1] = (uint32_t*)(scratch + n4);
+    a.vals[0] = (uint32_t*)(scratch + 2 * n4); a.vals[1] = (uint32_t*)(scratch + 3 * n4);
+    a.temp = scratch + 4 * n4;
+    const cudaError_t e = sort_launch(a, stream);
+    CUDA_TRY(cudaFreeAsync(scratch, stream));
+    CUDA_TRY(e);
+    return M2S_OK;
+}
+
+M2S_EXPORT m2s_status m2s_sort_quads(m2s_ctx* ctx, const void* d_quads, const float* d_depths, uint64_t count, void* d_sorted_quads,
+                                     uint32_t* d_order, float* device_ms) {
+    if (!ctx) { set_error("m2s_sort_quads: ctx is NULL"); return M2S_E_INVALID; }
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    m2s_status st = timing_events(ctx);
+    if (st != M2S_OK) return st;
+    CUDA_TRY(cudaEventRecord(ctx->ev_r[0], ctx->stream));
+    st = m2s_sort_quads_enqueue(ctx, d_quads, d_depths, count, nullptr, d_sorted_quads, d_order, ctx->stream);
+    if (st != M2S_OK) return st;
+    CUDA_TRY(cudaEventRecord(ctx->ev_r[1], ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    if (device_ms) CUDA_TRY(cudaEventElapsedTime(device_ms, ctx->ev_r[0], ctx->ev_r[1]));
+    return M2S_OK;
+}
+
+static m2s_status splat_validate(m2s_ctx* ctx, const void* d_sorted_quads, uint64_t count, const m2s_splat_params* p, const m2s_gbuffer* gb) {
+    if (!ctx || !p || !gb || (count && !d_sorted_quads) || !gb->position || !gb->normal || !gb->albedo || !gb->depth || !gb->metallic_roughness) {
+        set_error("m2s_splat: NULL argument"); return M2S_E_INVALID;
+    }
+    if (p->width < 1 || p->width > 4096 || p->height < 1 || p->height > 4096) { set_error("m2s_splat: width and height must be 1..4096"); return M2S_E_INVALID; }
+    if (p->render_mode == 3 || p->render_mode > 6) { set_error("m2s_splat: render modes 0-2 and 4-6 only"); return M2S_E_INVALID; }
+    if (count >= (1ull << 32)) { set_error("m2s_splat: too many quads (< 2^32 supported)"); return M2S_E_INVALID; }
+    if (misaligned16(d_sorted_quads) || misaligned16(gb->position) || misaligned16(gb->normal) || misaligned16(gb->albedo) ||
+        misaligned16(gb->depth) || misaligned16(gb->metallic_roughness)) {
+        set_error("m2s_splat: the quads and the G-buffer images must be 16-byte aligned"); return M2S_E_INVALID;
+    }
+    return M2S_OK;
+}
+
+static void splat_args(m2s_ctx* ctx, const void* d_sorted_quads, uint64_t count, const uint32_t* d_count, const m2s_splat_params* p,
+                       const m2s_gbuffer* gb, SplatArgs& a) {
+    std::memset(&a, 0, sizeof(a));
+    a.quads = (const float4*)d_sorted_quads; a.count = count; a.d_count = d_count;
+    a.width = (int)p->width; a.height = (int)p->height; a.mode = p->render_mode;
+    a.tiles_x = (a.width + kSplatTile - 1) / kSplatTile; a.tiles_y = (a.height + kSplatTile - 1) / kSplatTile;
+    a.position = (uint2*)gb->position; a.normal = (uint2*)gb->normal; a.depth = (uint2*)gb->depth;
+    a.albedo = (uint32_t*)gb->albedo; a.metallic_roughness = (uint32_t*)gb->metallic_roughness;
+    a.status = ctx->d_status;
+}
+
+static inline size_t up256(size_t b) { return (b + 255) & ~(size_t)255; }
+
+// scratch of the per-quad stage: records, tile counts, their scan, CUB temporary storage
+static m2s_status splat_alloc_prepare(SplatArgs& a, cudaStream_t stream, unsigned char** block) {
+    const size_t n = a.count ? a.count : 1;
+    const size_t tb = splat_scan_temp_bytes(n);
+    const size_t b_rec = up256(n * splat_rec_bytes()), b_tiles = up256(n * 4), b_incl = up256(n * 8);
+    CUDA_TRY(cudaMallocAsync((void**)block, b_rec + b_tiles + b_incl + tb, stream));
+    a.rec = *block; a.tiles = (uint32_t*)(*block + b_rec); a.incl = (unsigned long long*)(*block + b_rec + b_tiles);
+    a.temp = *block + b_rec + b_tiles + b_incl; a.temp_bytes = tb;
+    return M2S_OK;
+}
+// scratch of the pair stage: keys and values (double-buffered), tile ranges, CUB temporary storage
+static m2s_status splat_alloc_finish(SplatArgs& a, uint64_t max_pairs, cudaStream_t stream, unsigned char** block) {
+    const int tiles = a.tiles_x * a.tiles_y;
+    const size_t mp = max_pairs ? max_pairs : 1;
+    const size_t tb = splat_sort_temp_bytes(mp, tiles);
+    const size_t b_pair = up256(mp * 4), b_ranges = up256((size_t)tiles * 8);
+    CUDA_TRY(cudaMallocAsync((void**)block, 4 * b_pair + b_ranges + tb, stream));
+    for (int k = 0; k < 2; ++k) { a.keys[k] = (uint32_t*)(*block + k * b_pair); a.vals[k] = (uint32_t*)(*block + (2 + k) * b_pair); }
+    a.ranges = (uint2*)(*block + 4 * b_pair);
+    a.temp = *block + 4 * b_pair + b_ranges; a.temp_bytes = tb;
+    a.max_pairs = max_pairs;
+    return M2S_OK;
+}
+
+M2S_EXPORT m2s_status m2s_splat_enqueue(m2s_ctx* ctx, const void* d_sorted_quads, uint64_t count, const uint32_t* d_count,
+                                        const m2s_splat_params* p, const m2s_gbuffer* gb, uint64_t max_pairs, void* stream_) {
+    m2s_status st = splat_validate(ctx, d_sorted_quads, count, p, gb);
+    if (st != M2S_OK) return st;
+    if (max_pairs >= (1ull << 31)) { set_error("m2s_splat_enqueue: max_pairs must be below 2^31"); return M2S_E_INVALID; }
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    cudaStream_t stream = stream_ ? (cudaStream_t)stream_ : ctx->stream;
+    SplatArgs a;
+    splat_args(ctx, d_sorted_quads, count, d_count, p, gb, a);
+    unsigned char *b0 = nullptr, *b1 = nullptr;
+    if ((st = splat_alloc_prepare(a, stream, &b0)) != M2S_OK) return st;
+    cudaError_t e = splat_prepare(a, stream);
+    if (e == cudaSuccess) {
+        if ((st = splat_alloc_finish(a, max_pairs, stream, &b1)) != M2S_OK) { cudaFreeAsync(b0, stream); return st; }
+        e = splat_finish(a, stream);
+        CUDA_TRY(cudaFreeAsync(b1, stream));
+    }
+    CUDA_TRY(cudaFreeAsync(b0, stream));
+    CUDA_TRY(e);
+    return M2S_OK;
+}
+
+M2S_EXPORT m2s_status m2s_splat(m2s_ctx* ctx, const void* d_sorted_quads, uint64_t count, const uint32_t* d_count,
+                                const m2s_splat_params* p, const m2s_gbuffer* gb, uint64_t* pairs, float* device_ms) {
+    m2s_status st = splat_validate(ctx, d_sorted_quads, count, p, gb);
+    if (st != M2S_OK) return st;
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    if ((st = timing_events(ctx)) != M2S_OK) return st;
+    cudaStream_t stream = ctx->stream;
+    SplatArgs a;
+    splat_args(ctx, d_sorted_quads, count, d_count, p, gb, a);
+    unsigned char *b0 = nullptr, *b1 = nullptr;
+    if ((st = splat_alloc_prepare(a, stream, &b0)) != M2S_OK) return st;
+    CUDA_TRY(cudaEventRecord(ctx->ev_r[0], stream));
+    cudaError_t e = splat_prepare(a, stream);
+    unsigned long long total = 0;
+    if (e == cudaSuccess && count) e = cudaMemcpyAsync(ctx->h_total, a.incl + count - 1, 8, cudaMemcpyDeviceToHost, stream);
+    if (e == cudaSuccess) e = cudaEventRecord(ctx->ev_r[1], stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
+    if (e == cudaSuccess && count) total = *ctx->h_total;
+    if (e == cudaSuccess && total >= (1ull << 31)) {
+        cudaFreeAsync(b0, stream);
+        set_error("m2s_splat: more than 2^31 (tile, quad) pairs"); return M2S_E_CAPACITY;
+    }
+    if (e == cudaSuccess) {
+        if ((st = splat_alloc_finish(a, total, stream, &b1)) != M2S_OK) { cudaFreeAsync(b0, stream); return st; }
+        e = cudaEventRecord(ctx->ev_r[2], stream);
+        if (e == cudaSuccess) e = splat_finish(a, stream);
+        if (e == cudaSuccess) e = cudaEventRecord(ctx->ev_r[3], stream);
+        CUDA_TRY(cudaFreeAsync(b1, stream));
+    }
+    CUDA_TRY(cudaFreeAsync(b0, stream));
+    CUDA_TRY(e);
+    CUDA_TRY(cudaStreamSynchronize(stream));
+    if (pairs) *pairs = total;
+    if (device_ms) {
+        float t0 = 0.f, t1 = 0.f;
+        CUDA_TRY(cudaEventElapsedTime(&t0, ctx->ev_r[0], ctx->ev_r[1]));
+        CUDA_TRY(cudaEventElapsedTime(&t1, ctx->ev_r[2], ctx->ev_r[3]));
+        *device_ms = t0 + t1;
+    }
     return M2S_OK;
 }

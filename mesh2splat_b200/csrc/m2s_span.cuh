@@ -8,6 +8,7 @@
 // of O(width).  Used by raster_kernel (to count) and fragment_kernel (to enumerate); also compiled for the host
 // by tests/test_span_host.py (g++), which checks it against the brute-force per-pixel test.
 #pragma once
+#include <cmath>
 #include <cstdint>
 
 #if defined(__CUDACC__)
@@ -73,6 +74,74 @@ M2S_HD uint32_t span_row(const RowState& s, int yrel, int& xl) {
     }
     xl = lo;
     return hi >= lo ? (uint32_t)(hi - lo + 1) : 0u;
+}
+
+// The same rule for one pixel of the box: (xrel, yrel) relative to the box origin.
+M2S_HD bool span_covers(const RowState& s, int xrel, int yrel) {
+    bool in = true;
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+    for (int k = 0; k < 3; ++k) in = in && s.E[k] + (long long)s.A[k] * xrel + (long long)s.B[k] * yrel >= 0;
+    return in;
+}
+
+// fp32 operations without contraction, on the device and on the host (built with -ffp-contract=off there)
+M2S_HD float span_mul(float a, float b) {
+#if defined(__CUDA_ARCH__)
+    return __fmul_rn(a, b);
+#else
+    return a * b;
+#endif
+}
+M2S_HD float span_add(float a, float b) {
+#if defined(__CUDA_ARCH__)
+    return __fadd_rn(a, b);
+#else
+    return a + b;
+#endif
+}
+// Rasteriser set-up of one triangle given in normalised device coordinates (w = 1) for a W x H viewport at the origin
+// (GL 4.6 13.8.1, 14.6.1): xw = ndc * W/2 + W/2 in fp32 without contraction, snapped to 1/256 pixel; sign-normalised
+// edge functions with top-left ownership folded in; candidate box clamped to the viewport (which is also the clip:
+// GL clips to |x|, |y| <= w, exactly the pixels inside the viewport).  A corner that is not finite or lies beyond
+// the 8192-pixel guard band (the conversion's guard; the int32 edge steps need it) drops the triangle.  Returns false
+// if it cannot emit a fragment; else rs (relative to the box origin (x0, y0)) and the box height h.
+M2S_HD bool viewport_triangle_setup(const float ndx[3], const float ndy[3], int W, int H, RowState& rs, int& x0, int& y0, int& h) {
+    const float hw = (float)W * 0.5f, hh = (float)H * 0.5f;
+    int X[3], Y[3];
+    bool valid = true;
+    for (int k = 0; k < 3; ++k) {
+        const float xw = span_add(span_mul(ndx[k], hw), hw), yw = span_add(span_mul(ndy[k], hh), hh);
+        if (!(xw >= -8192.0f && xw <= 8192.0f) || !(yw >= -8192.0f && yw <= 8192.0f)) valid = false;   // also rejects NaN
+        X[k] = valid ? (int)rintf(span_mul(xw, 256.0f)) : 0;
+        Y[k] = valid ? (int)rintf(span_mul(yw, 256.0f)) : 0;
+    }
+    if (!valid) return false;
+    const long long area2 = (long long)(X[1] - X[0]) * (Y[2] - Y[0]) - (long long)(X[2] - X[0]) * (Y[1] - Y[0]);
+    if (area2 == 0) return false;
+    int xmin = X[0], xmax = X[0], ymin = Y[0], ymax = Y[0];
+    for (int k = 1; k < 3; ++k) {
+        xmin = X[k] < xmin ? X[k] : xmin; xmax = X[k] > xmax ? X[k] : xmax;
+        ymin = Y[k] < ymin ? Y[k] : ymin; ymax = Y[k] > ymax ? Y[k] : ymax;
+    }
+    int bx0 = (xmin + 127) >> 8, bx1 = (xmax - 128) >> 8, by0 = (ymin + 127) >> 8, by1 = (ymax - 128) >> 8;
+    bx0 = bx0 < 0 ? 0 : bx0; by0 = by0 < 0 ? 0 : by0;
+    bx1 = bx1 > W - 1 ? W - 1 : bx1; by1 = by1 > H - 1 ? H - 1 : by1;
+    if (bx1 < bx0 || by1 < by0) return false;
+    const int sg = area2 < 0 ? -1 : 1;
+    for (int k = 0; k < 3; ++k) {
+        const int va = (k + 1) % 3, vb = (k + 2) % 3;
+        const int dx = X[vb] - X[va], dy = Y[vb] - Y[va];
+        const int A = sg * (-dy * 256), B = sg * (dx * 256);
+        const long long C = (long long)sg * ((long long)dx * (128 - Y[va]) - (long long)dy * (128 - X[va]));
+        const bool owns = A > 0 || (A == 0 && B > 0);
+        rs.E[k] = C + (long long)A * bx0 + (long long)B * by0 - (owns ? 0 : 1);
+        rs.A[k] = A; rs.B[k] = B;
+    }
+    rs.w = bx1 - bx0 + 1;
+    x0 = bx0; y0 = by0; h = by1 - by0 + 1;
+    return true;
 }
 
 }  // namespace m2s
